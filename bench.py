@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- the hot path of rorosen/zeekstd (per-frame compress + decompress of a seekable archive) on B200.
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
   python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 ... bench.py --gpus N ...
 
 One STEP = compress a buffer into a seekable archive AND decompress that archive again (one pass of the hot path in both
@@ -26,6 +26,11 @@ bytes (the generator is counter-based: identical on CPU and GPU), frames spread 
 reaches (zeekstd itself is single-threaded) is reported beside it.  Both arms report the MEAN over the timed steps.
 `roofline.traffic` comes from the committed ncu capture named in `traffic_source`: a bench value is never taken under a
 profiler.
+
+--dump-outputs DIR writes, after the timed steps, what the last timed step handed its caller (rank 0's, at N > 1): archive.npy and
+output.npy (the compressed archive and the restored bytes, as float32, at fixed seeded positions when longer than 4 Mi bytes) and
+c_sizes.npy / d_sizes.npy (the seek table, float64).  The inputs depend only on the arguments, so two builds of the project can be
+compared output for output.
 """
 from __future__ import annotations
 
@@ -51,6 +56,8 @@ C4_REF_BYTES = int(os.environ.get("ZK_BENCH_C4_REF_BYTES", str(4 << 30)))   # bo
 C4_LEVEL, C4_SEED = 3, 20260925
 SEED = 20260924
 METRIC = "GiB/s compress + decompress (2 MiB frames)"
+DUMP_SEED = 20261017
+DUMP_SAMPLE = 1 << 22                      # bytes kept of each byte stream: 2 x 16 MiB of float32 in all
 KERNEL_NAMES = ["zk_scan_kernel", "zk_seq_kernel", "zk_huf_kernel", "zk_exec_kernel", "zk_xxh64_kernel", "zk_match_kernel",
                 "zk_entropy_enc_kernel", "zk_frame_*_kernels"]
 TRAFFIC_FILE = os.path.join(ROOT, "profiles", "traffic_r2.json")
@@ -134,6 +141,21 @@ def gen_mix(nbytes: int, seed: int, mix=None, device="cpu"):
     return parts[0] if len(parts) == 1 else torch.cat(parts)
 
 
+def byte_sample(buf, n: int) -> np.ndarray:
+    """buf[:n] (a uint8 tensor) as float32: every byte, or DUMP_SAMPLE bytes at seeded positions that depend only on n"""
+    import torch
+    idx = np.arange(n) if n <= DUMP_SAMPLE else np.sort(np.random.default_rng(DUMP_SEED).integers(0, n, DUMP_SAMPLE))
+    return buf[torch.from_numpy(idx).to(buf.device)].cpu().numpy().astype(np.float32)
+
+
+def dump_outputs(out_dir: str, archive, archive_len: int, c_sizes, d_sizes, output, output_len: int) -> None:
+    os.makedirs(out_dir, exist_ok=True)
+    arrays = {"archive": byte_sample(archive, archive_len), "output": byte_sample(output, output_len),
+              "c_sizes": np.asarray(c_sizes, dtype=np.float64), "d_sizes": np.asarray(d_sizes, dtype=np.float64)}
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
 def cpu_reference(data: np.ndarray, threads: int, level: int = LEVEL, checksum: bool = False):
     """the reference path on the host cores: libzstd through zeekstd's call sequence -> (seconds compress, seconds decompress, ratio)"""
     from oracle import oracle as O
@@ -188,7 +210,7 @@ def main_reference(args, rank, world, ncores):
         return 0
     import torch
     from oracle import oracle as O
-    W = max(args.warmup, 0); K = max(args.steps, 1)
+    W = max(args.warmup, 0); K = args.steps
     dev = "cuda" if torch.cuda.is_available() else "cpu"        # generation only (same bytes either way); nothing of ours runs here
     if args.gpus <= 1:
         data = gen_mix(WORKLOAD_BYTES, SEED, device=dev).cpu().numpy()
@@ -257,7 +279,7 @@ class Rig:
             rc = lib.zk_decompress_frames_dev(ctx._h, comp.data_ptr(), co.ctypes.data_as(N.u64p), do.ctypes.data_as(N.u64p), k, back.data_ptr(), int(checksum), None, None)
             assert rc == 0, rc
             return t_c, ctx.last_device_ms, int(co[-1])
-        step.back, step.cs, step.nf = back, cs, nf
+        step.comp, step.back, step.cs, step.ds, step.nf = comp, back, cs, ds, nf
         return step
 
     def timed_device(self, x, level, checksum, warmup, steps, dist=None):
@@ -424,7 +446,7 @@ def main_ours(args, rank, world, local, ncores):
         dist.init_process_group("nccl", device_id=torch.device("cuda", local), timeout=datetime.timedelta(seconds=180))   # a hang must fail fast
     rig = Rig(local)
     lib, ctx, dev = rig.lib, rig.ctx, rig.dev
-    W, K = max(args.warmup, 3), max(args.steps, 1)
+    W, K = max(args.warmup, 3), args.steps
     gib = 2.0**30
 
     # ---------------------------------------------------------------- configs[1] on this rank's GPU (headline at N = 1, `weak` at N > 1)
@@ -438,6 +460,9 @@ def main_ours(args, rank, world, local, ncores):
     launches = ctx.kernel_launches - launches0
     roof = roofline_block(rig, n + clen, n) if rank == 0 else None
     lib.zk_ctx_profile(ctx._h, 0)
+    if args.dump_outputs and world == 1:
+        s = rig.last_step
+        dump_outputs(args.dump_outputs, s.comp, clen, s.cs[: s.nf.value], s.ds[: s.nf.value], s.back, n)
     t = torch.tensor([tc_ms, td_ms], dtype=torch.float64, device=dev)
     if dist:
         dist.all_reduce(t, op=dist.ReduceOp.MAX)                                # device time, max over ranks
@@ -508,7 +533,7 @@ def main_ours(args, rank, world, local, ncores):
     dist.barrier(); torch.cuda.synchronize()
     tcs = tds = 0.0
     acc = {}
-    for _ in range(K):
+    for it in range(K):
         rig.flush.fill_(1); torch.cuda.synchronize(); dist.barrier()
         st = {}
         ev[0].record()
@@ -520,6 +545,8 @@ def main_ours(args, rank, world, local, ncores):
         for k_, v_ in st.items():
             acc[k_] = acc.get(k_, 0.0) + float(v_)
         clen4 = int(np.sum(cs))
+        if args.dump_outputs and rank == 0 and it == K - 1:
+            dump_outputs(args.dump_outputs, frames, clen4, cs, ds, back, nb)
         del frames, back
     torch.cuda.synchronize(); dist.barrier()
     clocks4 = sampler.result()
@@ -573,7 +600,12 @@ def main():
     ap.add_argument("--steps", type=int, default=5)
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the last timed step's outputs to DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes what this project's codec computed: it needs --impl ours")
     rank = int(os.environ.get("RANK", "0")); world = int(os.environ.get("WORLD_SIZE", "1")); local = int(os.environ.get("LOCAL_RANK", "0"))
     ncores = os.cpu_count() or 1
     if args.impl == "reference":
