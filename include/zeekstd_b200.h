@@ -120,6 +120,31 @@ int32_t zk_decompress_frames_prefix(zk_ctx* ctx, const uint8_t* comp, const uint
                                     int32_t* status, const uint8_t* prefix, size_t prefix_len);
 
 /*
+ * Context parameters (the ones the reference's CLI sets on its CCtx / DCtx for patch files, cli/src/compress.rs:31-37,
+ * cli/src/decompress.rs:53-62).  A zk_ctx plays both roles, so both kinds live on it.  They are sticky, like libzstd's, and apply
+ * to every batch and mirror call made on the context.  Value 0 restores the default.  Unknown parameter: ZK_ERR_ZSTD(40)
+ * (parameter_unsupported); value out of range: ZK_ERR_ZSTD(42) (parameter_outOfBound).
+ *
+ *   ZK_C_WINDOW_LOG (0, 10..30)          the Window_Descriptor announces max(the level's own window, 2^value); no offset the
+ *                                        encoder emits exceeds the announced window.  Values below a level's window change nothing.
+ *   ZK_C_ENABLE_LONG_DISTANCE_MATCHING   0 / 1.  Takes effect in prefix calls only: the part of the prefix the window reaches is
+ *   (0, 1)                               indexed on the device and every block of every frame searches it.  With window log 0 the
+ *                                        window is 2^27, as in libzstd.  Without a prefix it is a no-op for now (no in-frame
+ *                                        long-distance matching yet).
+ *   ZK_D_WINDOW_LOG_MAX (0, 10..30)      frames announcing a window above 2^value are refused (ZK_ERR_ZSTD(16)); default (0):
+ *                                        2^27 + 1, the limit of a default ZSTD_DCtx.
+ *
+ * Window logs stop at 30, one below libzstd's 64-bit maximum: the decoder keeps every concrete offset below 2^31.
+ */
+#define ZK_C_WINDOW_LOG 101                      /* = ZSTD_c_windowLog */
+#define ZK_C_ENABLE_LONG_DISTANCE_MATCHING 160   /* = ZSTD_c_enableLongDistanceMatching */
+#define ZK_D_WINDOW_LOG_MAX 100                  /* = ZSTD_d_windowLogMax */
+#define ZK_WINDOWLOG_MIN 10
+#define ZK_WINDOWLOG_MAX 30
+int32_t zk_ctx_set_cparameter(zk_ctx* ctx, int32_t param, int32_t value);
+int32_t zk_ctx_set_dparameter(zk_ctx* ctx, int32_t param, int32_t value);
+
+/*
  * Device-resident variants (zero-copy; used for roofline measurements and multi-GPU pipelines).
  * d_* are CUDA device pointers, 16-byte aligned, with >= 16 readable bytes after the last byte;
  * offset / size arrays stay on the HOST.  cuda_stream is a cudaStream_t (NULL = the context's own

@@ -95,6 +95,32 @@ class FrameSizePolicy:
     def default(cls): return cls.Uncompressed(0x200000)
 
 
+class CParameter:
+    """Compression parameters of a Context, named as zstd-safe's CParameter (ZSTD_c_* values).  0 restores the default."""
+    WINDOW_LOG = 101                      # ZK_C_WINDOW_LOG
+    ENABLE_LONG_DISTANCE_MATCHING = 160   # ZK_C_ENABLE_LONG_DISTANCE_MATCHING
+
+    def __init__(self, param: int, value: int):
+        self.param, self.value = param, int(value)
+
+    @classmethod
+    def WindowLog(cls, log: int): return cls(cls.WINDOW_LOG, log)
+
+    @classmethod
+    def EnableLongDistanceMatching(cls, on: bool): return cls(cls.ENABLE_LONG_DISTANCE_MATCHING, int(bool(on)))
+
+
+class DParameter:
+    """Decompression parameters of a Context, named as zstd-safe's DParameter (ZSTD_d_* values).  0 restores the default."""
+    WINDOW_LOG_MAX = 100                  # ZK_D_WINDOW_LOG_MAX
+
+    def __init__(self, param: int, value: int):
+        self.param, self.value = param, int(value)
+
+    @classmethod
+    def WindowLogMax(cls, log: int): return cls(cls.WINDOW_LOG_MAX, log)
+
+
 class Context:
     """Owns the CUDA streams / HBM scratch (the role CCtx / DCtx play in the reference)."""
 
@@ -103,6 +129,20 @@ class Context:
         h = c_void_p()
         _check(self.lib.zk_ctx_create(device, 0, byref(h)), self.lib)
         self._h = h
+        self.cparams: dict[int, int] = {}     # values set so far (sticky, as on the native context)
+        self.dparams: dict[int, int] = {}
+
+    def set_cparameter(self, p: CParameter) -> "Context":
+        """CCtx::set_parameter: applies to every later compress call on this context (window log 0 or 10..30, LDM 0/1)"""
+        _check(self.lib.zk_ctx_set_cparameter(self._h, p.param, p.value), self.lib)
+        self.cparams[p.param] = p.value
+        return self
+
+    def set_dparameter(self, p: DParameter) -> "Context":
+        """DCtx::set_parameter: applies to every later decompress call on this context (window log max 0 or 10..30)"""
+        _check(self.lib.zk_ctx_set_dparameter(self._h, p.param, p.value), self.lib)
+        self.dparams[p.param] = p.value
+        return self
 
     def close(self):
         if self._h:
@@ -587,7 +627,7 @@ class Decoder(io.RawIOBase):
         return int(v.value)
 
 
-__all__ = ["Context", "default_context", "set_default_context", "Error", "Format", "FrameSizePolicy", "SeekTable", "Serializer",
+__all__ = ["Context", "CParameter", "DParameter", "default_context", "set_default_context", "Error", "Format", "FrameSizePolicy", "SeekTable", "Serializer",
            "EncodeOptions", "RawEncoder", "Encoder", "CompressionProgress", "EpilogueProgress", "DecodeOptions", "Decoder",
            "BytesWrapper", "OffsetFrom", "SEEKABLE_MAGIC_NUMBER", "SEEKABLE_MAX_FRAMES", "SEEK_TABLE_INTEGRITY_SIZE",
            "SEEKABLE_MAX_FRAME_SIZE"]

@@ -50,6 +50,8 @@ _SIGS = {
     "zk_compress_bound": (c_size_t, [c_size_t, c_uint32]),
     "zk_ctx_profile": (None, [c_void_p, c_int32]),
     "zk_ctx_profile_read": (None, [c_void_p, POINTER(c_float), u32p]),
+    "zk_ctx_set_cparameter": (c_int32, [c_void_p, c_int32, c_int32]),
+    "zk_ctx_set_dparameter": (c_int32, [c_void_p, c_int32, c_int32]),
     "zk_compress_frames": (c_int32, [c_void_p, c_void_p, c_size_t, c_uint32, c_int32, c_int32, c_void_p, c_size_t,
                                      u32p, u32p, c_uint32, u32p, POINTER(c_size_t)]),
     "zk_decompress_frames": (c_int32, [c_void_p, c_void_p, u64p, u64p, c_uint32, c_void_p, c_int32, i32p]),

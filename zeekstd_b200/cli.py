@@ -8,8 +8,11 @@ What each piece follows in the reference: argument set and value parsers cli/src
 path derivation, overwrite checks and the list tables cli/src/command.rs:33-473; the compress loop (Encoder fed from a
 reader, optional stand-alone Head-format seek table) cli/src/compress.rs:55-106; the decompress loop
 cli/src/decompress.rs:21-117.  The codec underneath is this package's Encoder / Decoder, i.e. the CUDA path: there is no
-CPU route.  The window-log / long-distance-matching parameters the reference sets for patch files have no counterpart
-here (the kernels take the prefix as it is); `--mmap-prefix` / `--no-mmap-prefix` choose between np.memmap and a read.
+CPU route.  Patch files get the parameters the reference sets (compress.rs:31-37, decompress.rs:53-62): `--patch-from`
+sets window log clamp(ilog2(len) + 1, 17, 30) and long-distance matching, so matches reach anywhere in the window's part of
+the prefix; `--patch-apply` raises the decoder's window limit to 2^max(27, ilog2(len) + 1) (at most 2^30) -- never below
+the default, since this encoder's frames announce at least 128 KiB.  `--mmap-prefix` / `--no-mmap-prefix` choose between
+np.memmap and a read.
 """
 from __future__ import annotations
 
@@ -351,6 +354,34 @@ def _run_compress(zk, ns, fmt_bytes) -> int:
     return 0
 
 
+def _patch_window_log(prefix_len: int, floor: int) -> int:
+    """ilog2(len) + 1 (cli/src/compress.rs:31-37), between `floor` and 30 (the largest window log of this codec)"""
+    return min(30, max(floor, max(prefix_len, 1).bit_length()))
+
+
+class _ContextParams:
+    """sets context parameters for one command and restores the previous values afterwards (the context outlives the command)"""
+
+    def __init__(self, ctx, cparams=(), dparams=()):
+        self.ctx, self.cparams, self.dparams = ctx, list(cparams), list(dparams)
+
+    def __enter__(self):
+        self.saved = (dict(self.ctx.cparams), dict(self.ctx.dparams))
+        for p in self.cparams:
+            self.ctx.set_cparameter(p)
+        for p in self.dparams:
+            self.ctx.set_dparameter(p)
+        return self
+
+    def __exit__(self, *exc):
+        import zeekstd_b200 as zk
+        for p in self.cparams:
+            self.ctx.set_cparameter(zk.CParameter(p.param, self.saved[0].get(p.param, 0)))
+        for p in self.dparams:
+            self.ctx.set_dparameter(zk.DParameter(p.param, self.saved[1].get(p.param, 0)))
+        return False
+
+
 def _run_decompress(zk, ns, fmt_bytes) -> int:
     in_path = ns.input_file
     out_path = _out_path(ns, in_path)
@@ -460,9 +491,15 @@ def main(argv=None) -> int:
     fmt_bytes = raw_bytes if ns.raw_bytes else human_bytes
     try:
         if ns.command == "compress":
-            return _run_compress(zk, ns, fmt_bytes)
+            n = os.path.getsize(ns.patch_from) if ns.patch_from and os.path.exists(ns.patch_from) else None
+            cp = [] if n is None else [zk.CParameter.WindowLog(_patch_window_log(n, 17)), zk.CParameter.EnableLongDistanceMatching(True)]
+            with _ContextParams(zk.default_context(), cparams=cp):
+                return _run_compress(zk, ns, fmt_bytes)
         if ns.command == "decompress":
-            return _run_decompress(zk, ns, fmt_bytes)
+            n = os.path.getsize(ns.patch_apply) if ns.patch_apply and os.path.exists(ns.patch_apply) else None
+            dp = [] if n is None else [zk.DParameter.WindowLogMax(_patch_window_log(n, 27))]
+            with _ContextParams(zk.default_context(), dparams=dp):
+                return _run_decompress(zk, ns, fmt_bytes)
         return _run_list(zk, ns, fmt_bytes)
     except CliError as e:
         sys.stderr.write(f"Error: {e}\n")

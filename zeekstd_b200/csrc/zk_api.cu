@@ -61,6 +61,7 @@ extern "C" const char* zk_error_name(int32_t rc) {
     case -22: return "Restored data doesn't match checksum";
     case -30: return "Dictionary is corrupted";
     case -32: return "Dictionary mismatch";
+    case -40: return "Unsupported parameter";
     case -42: return "Parameter is out of bound";
     case -64: return "Allocation error : not enough memory";
     case -70: return "Destination buffer is too small";
@@ -140,9 +141,33 @@ extern "C" void zk_ctx_destroy(zk_ctx* c) {
     if (c->up) cudaStreamDestroy(c->up);
     if (c->down) cudaStreamDestroy(c->down);
     if (c->d_prefix) cudaFree(c->d_prefix);
+    if (c->d_ldm) cudaFree(c->d_ldm);
     if (c->ev0) cudaEventDestroy(c->ev0);
     if (c->ev1) cudaEventDestroy(c->ev1);
     delete c;
+}
+
+// context parameters (include/zeekstd_b200.h): sticky, 0 = default
+extern "C" int32_t zk_ctx_set_cparameter(zk_ctx* c, int32_t param, int32_t value) {
+    if (!c) return ZK_ERR_INVALID_ARG;
+    switch (param) {
+    case ZK_C_WINDOW_LOG:
+        if (value != 0 && (value < ZK_WINDOWLOG_MIN || value > ZK_WINDOWLOG_MAX)) return ZK_ERR_ZSTD(ZKZ_PARAM_OUT_OF_BOUND);
+        c->c_window_log = value; return 0;
+    case ZK_C_ENABLE_LONG_DISTANCE_MATCHING:
+        if (value != 0 && value != 1) return ZK_ERR_ZSTD(ZKZ_PARAM_OUT_OF_BOUND);
+        c->c_ldm = value; return 0;
+    default: return ZK_ERR_ZSTD(ZKZ_PARAM_UNSUPPORTED);
+    }
+}
+
+extern "C" int32_t zk_ctx_set_dparameter(zk_ctx* c, int32_t param, int32_t value) {
+    if (!c) return ZK_ERR_INVALID_ARG;
+    if (param != ZK_D_WINDOW_LOG_MAX) return ZK_ERR_ZSTD(ZKZ_PARAM_UNSUPPORTED);
+    if (value != 0 && (value < ZK_WINDOWLOG_MIN || value > ZK_WINDOWLOG_MAX)) return ZK_ERR_ZSTD(ZKZ_PARAM_OUT_OF_BOUND);
+    c->d_window_log_max = value;
+    for (int i = 0; i < ZK_SLOTS; i++) c->slot[i].dws.win_max = value ? 1ull << value : (1ull << 27) + 1;
+    return 0;
 }
 
 extern "C" uint64_t zk_ctx_kernel_launches(const zk_ctx* c) { return c ? c->launches() : 0; }
@@ -340,6 +365,7 @@ extern "C" int32_t zk_compress_frames_dev(zk_ctx* c, const void* d_src, size_t n
         const size_t in_len = n - in_off < (size_t)cnt * frame_size ? n - in_off : (size_t)cnt * frame_size;
         size_t produced = 0;
         c->slot[0].ews.no_side = false;
+        c->slot[0].ews.win_log = (uint32_t)c->c_window_log;
         int rc = zk_encode_batch(&c->slot[0].ews, st, (const uint8_t*)d_src + in_off, in_len, frame_size, level, checksum,
                                  (uint8_t*)d_dst + out_pos, dst_cap - out_pos, c_sizes ? c_sizes + f0 : nullptr, cnt, &produced);
         if (rc) return rc;
@@ -412,6 +438,8 @@ extern "C" int32_t zk_compress_frames(zk_ctx* c, const uint8_t* src, size_t n, u
         tr.mark(s.stream, (int)k, 1);
         s.ews.no_side = zk_env_size("ZK_HOST_SIDE", 1) == 0;
         s.ews.prefix = c->cur_prefix_len ? c->d_prefix : nullptr; s.ews.prefix_len = c->cur_prefix_len;
+        s.ews.ldm_tab = c->cur_prefix_len && c->cur_ldm_log ? c->d_ldm : nullptr; s.ews.ldm_log = c->cur_ldm_log;
+        s.ews.win_log = c->cur_ldm_win ? c->cur_ldm_win : (uint32_t)c->c_window_log;
         rc = zk_encode_enqueue(&s.ews, s.stream, s.d_in, sb.in_len, frame_size, level, checksum, s.d_out, bound, sb.cnt);
         if (rc) { err = rc; break; }
         tr.mark(s.stream, (int)k, 2);
@@ -465,8 +493,25 @@ extern "C" int32_t zk_compress_frames_prefix(zk_ctx* c, const uint8_t* src, size
     if (!c) return ZK_ERR_INVALID_ARG;
     int32_t rc = zk_ctx_set_prefix(c, prefix, prefix_len);
     if (rc) return rc;
+    if (c->c_ldm && c->cur_prefix_len && n) {
+        // long-distance matching: index the part of the prefix the window reaches (window log 27 unless set, as libzstd)
+        const uint32_t wl = c->c_window_log ? (uint32_t)c->c_window_log : 27u, tl = zk_encode_level_window_log(level);
+        const uint32_t win_log = wl > tl ? wl : tl;
+        const size_t span = c->cur_prefix_len < (1ull << win_log) ? c->cur_prefix_len : (size_t)1 << win_log;
+        const uint32_t log = zk_ldm_index_log(span);
+        if (c->cap_ldm < ((size_t)4 << log)) {
+            if (c->d_ldm) cudaFree(c->d_ldm);
+            c->d_ldm = nullptr; c->cap_ldm = 0;
+            if (cudaMalloc((void**)&c->d_ldm, (size_t)4 << log) != cudaSuccess) { c->cur_prefix_len = 0; return ZK_ERR_ZSTD(ZKZ_MEMORY_ALLOCATION); }
+            c->cap_ldm = (size_t)4 << log;
+        }
+        rc = zk_ldm_index_build(c->slot[0].stream, c->d_prefix, c->cur_prefix_len, 1u << win_log, c->d_ldm, log);
+        if (!rc && cudaStreamSynchronize(c->slot[0].stream) != cudaSuccess) rc = ZK_ERR_CUDA;
+        if (rc) { c->cur_prefix_len = 0; return rc == ZK_INT_CUDA ? ZK_ERR_CUDA : rc; }
+        c->cur_ldm_log = log; c->cur_ldm_win = win_log;
+    }
     rc = zk_compress_frames(c, src, n, frame_size, level, checksum, dst, dst_cap, c_sizes, d_sizes, frames_cap, n_frames, dst_len);
-    c->cur_prefix_len = 0;
+    c->cur_prefix_len = 0; c->cur_ldm_log = 0; c->cur_ldm_win = 0;
     return rc;
 }
 

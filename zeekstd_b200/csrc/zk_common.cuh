@@ -63,6 +63,7 @@ enum ZkZstdCode : int {
     ZKZ_CHECKSUM_WRONG = 22,
     ZKZ_DICT_CORRUPTED = 30,         // what libzstd reports for Treeless literals before any Huffman table (litEntropy == 0)
     ZKZ_DICT_WRONG = 32,
+    ZKZ_PARAM_UNSUPPORTED = 40,
     ZKZ_PARAM_OUT_OF_BOUND = 42,
     ZKZ_MEMORY_ALLOCATION = 64,
     ZKZ_DST_TOO_SMALL = 70,

@@ -23,6 +23,11 @@ struct zk_ctx {
     float last_ms = 0.f;
     uint8_t* d_prefix = nullptr; size_t cap_prefix = 0;   // device copy of the raw-content prefix of the *_prefix entry points
     uint32_t cur_prefix_len = 0;                          // != 0 while such a call is running: every sub-batch gets the prefix
+    // context parameters (zk_ctx_set_cparameter / zk_ctx_set_dparameter); 0 = default
+    int32_t c_window_log = 0, c_ldm = 0, d_window_log_max = 0;
+    // long-distance-matching index of the prefix (zk_ldm_index_build): 2^ldm_log u32 slots, grown on demand
+    uint32_t* d_ldm = nullptr; size_t cap_ldm = 0;
+    uint32_t cur_ldm_log = 0, cur_ldm_win = 0;            // != 0 while a prefix call with LDM runs: index log, window log
     unsigned long long launches() const {
         unsigned long long n = 0;
         for (int i = 0; i < ZK_SLOTS; i++) n += slot[i].dws.launches + slot[i].ews.launches;

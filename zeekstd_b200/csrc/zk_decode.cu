@@ -64,7 +64,7 @@ __device__ __forceinline__ uint32_t zk_parse_nseq(const uint8_t* s, uint32_t n, 
 
 // Walks every zstd / skippable frame inside one seek-table entry.  emit(info) is called per block.
 template <class Emit>
-__device__ int zk_walk_entry(const uint8_t* p, uint32_t n, Emit& emit) {
+__device__ int zk_walk_entry(const uint8_t* p, uint32_t n, Emit& emit, unsigned long long win_max) {
     uint32_t pos = 0;
     while (pos < n) {
         if (n - pos < 4) return ZKZ_SRC_SIZE_WRONG;
@@ -100,9 +100,10 @@ __device__ int zk_walk_entry(const uint8_t* p, uint32_t n, Emit& emit) {
         for (uint32_t i = 0; i < fcs_sz; i++) fcs |= (unsigned long long)p[q + i] << (8 * i);
         if (fcs_sz == 2) fcs += 256;
         // the reference decodes with a default DCtx (decode.rs:130-133): streaming decompression refuses windows above
-        // 2^ZSTD_WINDOWLOG_LIMIT_DEFAULT (+1), after the dictionary check -- a Single_Segment frame's window is its content size
+        // 2^ZSTD_WINDOWLOG_LIMIT_DEFAULT (+1), after the dictionary check -- a Single_Segment frame's window is its content size.
+        // ZK_D_WINDOW_LOG_MAX moves the limit to 2^value, as ZSTD_d_windowLogMax does
         if (single) window = fcs;
-        if (window > (1ull << 27) + 1) return ZKZ_WINDOW_TOO_LARGE;
+        if (window > win_max) return ZKZ_WINDOW_TOO_LARGE;
         // Block_Maximum_Size = min(Window_Size, 128 KiB) (RFC 8878 3.1.1.2.3): libzstd refuses a block whose content or
         // regenerated size exceeds it (ZSTD_decompressContinue: "Block Size Exceeds Maximum", "Decompressed Block Size Exceeds Maximum")
         const uint32_t bsmax = window < ZK_BLOCK_MAX ? (uint32_t)window : ZK_BLOCK_MAX;
@@ -217,7 +218,7 @@ __global__ void __launch_bounds__(128) zk_scan_kernel(ZkDecodeArgs a) {
     if (c1 < c0 || c1 - c0 > 0xFFFFFFFFull) { ent.status = -ZKZ_SRC_SIZE_WRONG; a.entries[e] = ent; return; }
     const uint8_t* p = a.comp + c0; uint32_t n = (uint32_t)(c1 - c0);
     ZkCountEmit ce;
-    int rc = zk_walk_entry(p, n, ce);
+    int rc = zk_walk_entry(p, n, ce, a.win_max);
     if (rc) { ent.status = -rc; atomicAdd(&a.counters->n_errors, 1u); a.entries[e] = ent; return; }
     unsigned long long b0 = atomicAdd(&a.counters->n_blocks, (unsigned long long)ce.nb);
     unsigned long long l0 = atomicAdd(&a.counters->n_lit, (unsigned long long)ce.nlit);
@@ -229,7 +230,7 @@ __global__ void __launch_bounds__(128) zk_scan_kernel(ZkDecodeArgs a) {
     }
     ZkFillEmit fe; fe.blocks = a.blocks; fe.entry = e; fe.bidx = (uint32_t)b0; fe.lit = (uint32_t)l0; fe.seq = (uint32_t)s0;
     fe.ebase = p; fe.huf_list = a.huf_list; fe.seq_list = a.seq_list; fe.hufi = h0; fe.sqbi = q0;   // lists have cap_blocks entries
-    rc = zk_walk_entry(p, n, fe);
+    rc = zk_walk_entry(p, n, fe, a.win_max);
     ent.first_block = (uint32_t)b0; ent.n_blocks = ce.nb;
     if (rc) { ent.status = -rc; ent.n_blocks = 0; atomicAdd(&a.counters->n_errors, 1u); }
     a.entries[e] = ent;
@@ -2084,6 +2085,7 @@ int zk_decode_enqueue(ZkDecodeWs* ws, cudaStream_t stream, const uint8_t* d_comp
     a.cap_blocks = ws->cap_blocks; a.cap_lit = ws->cap_lit - 64; a.cap_seq = ws->cap_seq;
     a.trace = nullptr;
     a.d_need = nullptr;
+    a.win_max = ws->win_max;
     a.prefix = ws->prefix; a.prefix_len = ws->prefix ? ws->prefix_len : 0; ws->prefix = nullptr; ws->prefix_len = 0;
     if (ws->need) {
         memcpy(ws->h_need, ws->need, (size_t)n * 4);

@@ -16,6 +16,7 @@ struct ZkDecodeArgs {                 // kernel parameter block (by value)
     unsigned long long* trace;        // debug: per-chunk clock64 stamps of entry 0 (env ZK_EXEC_TRACE), else nullptr
     const uint8_t* prefix; uint32_t prefix_len;   // raw-content prefix of every zstd frame (Decoder::decompress_with_prefix, decode.rs:211-214, 246-255); device pointer or nullptr
     const uint32_t* d_need;           // per entry: only this many leading bytes are wanted (range reads); nullptr = everything
+    unsigned long long win_max;       // frames announcing a larger window are refused (window_tooLarge)
 };
 
 struct ZkDecodeWs {                   // HBM scratch owned by a zk_ctx, grown on demand, reused across batches
@@ -45,6 +46,7 @@ struct ZkDecodeWs {                   // HBM scratch owned by a zk_ctx, grown on
     size_t want_blocks = 0, want_lit = 0, want_seq = 0;   // exact needs reported by a batch that overflowed
     uint32_t pending_n = 0;
     int sm_count = 0;
+    unsigned long long win_max = (1ull << 27) + 1;   // ZK_D_WINDOW_LOG_MAX of the owning context; default: a default ZSTD_DCtx's limit
     unsigned long long launches = 0;  // kernels launched so far (bench.py's gpu_launches)
     ZkProf prof;
 };

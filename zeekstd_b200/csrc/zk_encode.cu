@@ -50,6 +50,9 @@ struct ZkEncodeArgs {
     // ptail <= ZKC_BLOCK bytes of it are staged in front of a copy of each frame's first block, so that block's match finder sees
     // one contiguous history and needs no second pointer
     const uint8_t* prefix; uint32_t prefix_len, ptail; uint8_t* pstage;
+    // long-distance matching (the LDM flavour of K-C1 only): index of the prefix (zk_ldm_index_kernel) with 2^ldm_log slots, and the
+    // announced window -- no offset may exceed it
+    const uint32_t* ldm_tab; uint32_t ldm_log, ldm_win;
 };
 #define ZKC_PSLOT (2u * ZKC_BLOCK + 64u)   // per-frame staging slot: [prefix tail | first block]
 
@@ -77,6 +80,9 @@ __device__ __forceinline__ uint32_t zkc_hash5(unsigned long long v) {
 template <int HLOG>
 __device__ __forceinline__ uint32_t zkc_hash8(unsigned long long v) {
     return (uint32_t)((v * 0xCF1BBCDCB7A56463ull) >> (64 - HLOG));
+}
+__device__ __forceinline__ uint32_t zkc_ldm_hash(unsigned long long v, uint32_t log) {
+    return (uint32_t)((v * 0x9E3779B97F4A7C15ull) >> (64 - log));
 }
 
 // =============================================================================================
@@ -106,7 +112,9 @@ __global__ void __launch_bounds__(256) zk_prefix_stage_kernel(ZkEncodeArgs a) {
 
 // DFAST (level >= 4): a second table indexed by a hash of EIGHT bytes is probed first -- its candidates are long matches by
 // construction, the 5-byte table catches the rest (the idea of zstd's double-fast strategy); two tables of 2^HLOG entries per warp.
-template <int HLOG, int NW, bool DFAST>
+// LDM (long-distance matching, prefix calls with ZK_C_ENABLE_LONG_DISTANCE_MATCHING): every lane also probes the HBM index of the prefix
+// with the 8 bytes it holds; a verified hit becomes a match whose source lies anywhere in the prefix the window reaches.
+template <int HLOG, int NW, bool DFAST, bool LDM = false>
 __global__ void __launch_bounds__(NW * 32) zk_match_kernel(ZkEncodeArgs a) {
     __shared__ uint16_t tables[NW][(DFAST ? 2 : 1) << HLOG];
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
@@ -128,7 +136,7 @@ __global__ void __launch_bounds__(NW * 32) zk_match_kernel(ZkEncodeArgs a) {
 #define ZKC_WIDE_LEVEL 13
 #define ZKC_WIDE_HIST 7
 #define ZKC_WIDE_HLOG 15
-template <int HLOG>
+template <int HLOG, bool LDM = false>
 __global__ void __launch_bounds__(32) zk_match_wide_kernel(ZkEncodeArgs a) {
     ZK_DYN_SMEM(wide_tab);
     constexpr bool DFAST = false;
@@ -950,6 +958,22 @@ __global__ void __launch_bounds__(128) zk_frame_window_kernel(ZkEncodeArgs a, ui
     a.dst[a.frame_off[f] + 5] = 0x40;
 }
 
+// ZK_C_WINDOW_LOG / long-distance matching: the Window_Descriptor of every frame becomes 2^log (exponent log - 10, mantissa 0)
+__global__ void __launch_bounds__(128) zk_frame_wlog_kernel(ZkEncodeArgs a, uint32_t n_frames, uint32_t log) {
+    const uint32_t f = blockIdx.x * blockDim.x + threadIdx.x;
+    if (f >= n_frames || *a.error) return;
+    a.dst[a.frame_off[f] + 5] = (uint8_t)((log - 10u) << 3);
+}
+
+// long-distance matching: the index of the prefix.  One thread per sampled position q (every ZK_LDM_STRIDE-th position from q0 on);
+// atomicMax keeps the highest position per slot whatever the schedule, so the table -- and the compressed bytes -- are deterministic
+__global__ void __launch_bounds__(256) zk_ldm_index_kernel(const uint8_t* prefix, uint32_t q0, uint32_t count, uint32_t* tab, uint32_t log) {
+    const uint32_t i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= count) return;
+    const uint32_t q = q0 + i * ZK_LDM_STRIDE;
+    atomicMax(&tab[zkc_ldm_hash(zkc_ld8(prefix + q), log)], q + 1u);
+}
+
 // gather: one warp per block copies its staged bytes to the final position; block 0 of a frame also writes the
 // frame header, the last block the checksum
 __global__ void __launch_bounds__(128) zk_frame_gather_kernel(ZkEncodeArgs a) {
@@ -998,6 +1022,27 @@ __global__ void __launch_bounds__(128) zk_frame_gather_kernel(ZkEncodeArgs a) {
 #define ZKC_CUDA_OK(x) do { (void)(x); } while (0)
 #endif
 
+uint32_t zk_encode_level_window_log(int level) { return (level <= 0 ? 3 : level) >= ZKC_WIDE_LEVEL ? 18u : 17u; }
+
+// about one slot per sampled position, at least 2^12 and at most 2^26 slots (256 MiB, a 1 GiB window)
+uint32_t zk_ldm_index_log(size_t span) {
+    const size_t samples = span / ZK_LDM_STRIDE + 1;
+    uint32_t log = 12;
+    while (log < 26 && ((size_t)1 << log) < samples) log++;
+    return log;
+}
+
+int zk_ldm_index_build(cudaStream_t stream, const uint8_t* d_prefix, uint32_t prefix_len, uint32_t win, uint32_t* d_tab, uint32_t log) {
+    ZKC_CUDA_OK(cudaMemsetAsync(d_tab, 0, sizeof(uint32_t) << log, stream));
+    if (prefix_len < 8) return 0;
+    const uint32_t lo = prefix_len > win ? prefix_len - win : 0u;
+    const uint32_t q0 = (lo + ZK_LDM_STRIDE - 1) / ZK_LDM_STRIDE * ZK_LDM_STRIDE;
+    if (q0 > prefix_len - 8) return 0;
+    const uint32_t count = (prefix_len - 8 - q0) / ZK_LDM_STRIDE + 1;
+    ZK_LAUNCH(zk_ldm_index_kernel, (count + 255) / 256, 256, 0, stream, d_prefix, q0, count, d_tab, log);
+    return 0;
+}
+
 size_t zk_encode_bound(size_t n, uint32_t frame_size) {
     if (frame_size == 0) frame_size = 1;
     size_t frames = n / frame_size + 1;
@@ -1021,7 +1066,8 @@ static size_t zkc_align(size_t v) { return (v + 255) & ~(size_t)255; }
 int zk_encode_enqueue(ZkEncodeWs* ws, cudaStream_t stream, const uint8_t* d_src, size_t n, uint32_t frame_size, int level,
                       int checksum, uint8_t* d_dst, size_t dst_cap, uint32_t n_frames) {
     const uint8_t* d_prefix = ws->prefix; const uint32_t prefix_len = ws->prefix_len;     // one-shot (set by the caller for THIS batch)
-    ws->prefix = nullptr; ws->prefix_len = 0;
+    const uint32_t* ldm_tab = ws->ldm_tab; const uint32_t ldm_log = ws->ldm_log;
+    ws->prefix = nullptr; ws->prefix_len = 0; ws->ldm_tab = nullptr; ws->ldm_log = 0;
     ws->pending_frames = 0;
     if (n_frames == 0) return 0;
     if (frame_size == 0 || frame_size > 0x40000000u) return -(int)ZKZ_PARAM_OUT_OF_BOUND;
@@ -1067,6 +1113,11 @@ int zk_encode_enqueue(ZkEncodeWs* ws, cudaStream_t stream, const uint8_t* d_src,
     a.frame_csize = (uint32_t*)(base + o_fcs); a.frame_off = (unsigned long long*)(base + o_foff); a.frame_hash = (uint32_t*)(base + o_fh);
     a.dst = d_dst; a.dst_cap = dst_cap; a.total = (unsigned long long*)(base + o_tot); a.error = (uint32_t*)(base + o_tot + 8);
     a.prefix = d_prefix; a.prefix_len = 0; a.ptail = 0; a.pstage = base + o_pst;
+    // announced window: the level's own, raised to 2^win_log; the LDM flavour of K-C1 keeps every offset within it
+    const uint32_t tier_log = zk_encode_level_window_log(a.level);
+    const uint32_t win_log = ws->win_log > tier_log ? ws->win_log : tier_log;
+    const bool ldm = ldm_tab && d_prefix && prefix_len && n;
+    a.ldm_tab = ldm ? ldm_tab : nullptr; a.ldm_log = ldm ? ldm_log : 0; a.ldm_win = 1u << win_log;
     if (d_prefix && prefix_len && n) {
         a.prefix_len = prefix_len; a.ptail = prefix_len < ZKC_BLOCK ? prefix_len : ZKC_BLOCK;
         ZK_LAUNCH(zk_prefix_stage_kernel, n_frames, 256, 0, stream, a);
@@ -1094,7 +1145,19 @@ int zk_encode_enqueue(ZkEncodeWs* ws, cudaStream_t stream, const uint8_t* d_src,
     // previous-block history, one lazy step; 4-6 = double table (8-byte + 5-byte hashes, 4096 entries each), two warps per CTA; 7-9 = double
     // table of 8192 entries each, one warp per CTA; 10-12 = one table of 16384 entries, one warp per CTA; >= 13 = 256 KiB history, 32768 x u32
     // entries in dynamic shared memory.  Ratio on the reference's corpus: 2.12 / 2.24 / 2.28 / 2.38 / 2.40 / 2.50 (profiles/ratio_dickens_r2.json)
-    if (a.level <= 1) ZK_LAUNCH((zk_match_kernel<ZKC_HLOG_FAST, ZKC_C1_WARPS, false>), (uint32_t)((n_blocks + ZKC_C1_WARPS - 1) / ZKC_C1_WARPS), ZKC_C1_WARPS * 32, 0, stream, a);
+    if (ldm) {
+        if (a.level <= 1) ZK_LAUNCH((zk_match_kernel<ZKC_HLOG_FAST, ZKC_C1_WARPS, false, true>), (uint32_t)((n_blocks + ZKC_C1_WARPS - 1) / ZKC_C1_WARPS), ZKC_C1_WARPS * 32, 0, stream, a);
+        else if (a.level <= 3) ZK_LAUNCH((zk_match_kernel<ZKC_HLOG, ZKC_C1_WARPS, false, true>), (uint32_t)((n_blocks + ZKC_C1_WARPS - 1) / ZKC_C1_WARPS), ZKC_C1_WARPS * 32, 0, stream, a);
+        else if (a.level <= 6) ZK_LAUNCH((zk_match_kernel<ZKC_HLOG, 2, true, true>), (uint32_t)((n_blocks + 1) / 2), 64, 0, stream, a);
+        else if (a.level <= 9) ZK_LAUNCH((zk_match_kernel<13, 1, true, true>), (uint32_t)n_blocks, 32, 0, stream, a);
+        else if (a.level < ZKC_WIDE_LEVEL) ZK_LAUNCH((zk_match_kernel<14, 1, false, true>), (uint32_t)n_blocks, 32, 0, stream, a);
+        else {
+            const int wide_smem = (int)sizeof(uint32_t) << ZKC_WIDE_HLOG;
+            if (!ws->attr_set_wide_ldm) { ZKC_CUDA_OK(cudaFuncSetAttribute(zk_match_wide_kernel<ZKC_WIDE_HLOG, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, wide_smem)); ws->attr_set_wide_ldm = true; }
+            ZK_LAUNCH((zk_match_wide_kernel<ZKC_WIDE_HLOG, true>), (uint32_t)n_blocks, 32, wide_smem, stream, a);
+        }
+    }
+    else if (a.level <= 1) ZK_LAUNCH((zk_match_kernel<ZKC_HLOG_FAST, ZKC_C1_WARPS, false>), (uint32_t)((n_blocks + ZKC_C1_WARPS - 1) / ZKC_C1_WARPS), ZKC_C1_WARPS * 32, 0, stream, a);
     else if (a.level <= 3) ZK_LAUNCH((zk_match_kernel<ZKC_HLOG, ZKC_C1_WARPS, false>), (uint32_t)((n_blocks + ZKC_C1_WARPS - 1) / ZKC_C1_WARPS), ZKC_C1_WARPS * 32, 0, stream, a);
     else if (a.level <= 6) ZK_LAUNCH((zk_match_kernel<ZKC_HLOG, 2, true>), (uint32_t)((n_blocks + 1) / 2), 64, 0, stream, a);
     else if (a.level <= 9) ZK_LAUNCH((zk_match_kernel<13, 1, true>), (uint32_t)n_blocks, 32, 0, stream, a);
@@ -1122,6 +1185,7 @@ int zk_encode_enqueue(ZkEncodeWs* ws, cudaStream_t stream, const uint8_t* d_src,
     ZK_LAUNCH(zk_frame_scan_kernel, 1, 1024, 0, stream, a);
     ZK_LAUNCH(zk_frame_gather_kernel, (uint32_t)((n_blocks + 3) / 4), 128, 0, stream, a);
     if (a.level >= ZKC_WIDE_LEVEL) { ZK_LAUNCH(zk_frame_window_kernel, (n_frames + 127) / 128, 128, 0, stream, a, n_frames); ws->launches++; }
+    if (win_log > tier_log) { ZK_LAUNCH(zk_frame_wlog_kernel, (n_frames + 127) / 128, 128, 0, stream, a, n_frames, win_log); ws->launches++; }
     ws->prof.end(7, stream);
     ZKC_CUDA_OK(cudaMemcpyAsync(ws->h_sizes, a.frame_csize, (size_t)n_frames * 4, cudaMemcpyDeviceToHost, stream));
     ZKC_CUDA_OK(cudaMemcpyAsync(ws->h_sizes + ws->cap_frames, a.total, 16, cudaMemcpyDeviceToHost, stream));
